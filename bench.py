@@ -6,6 +6,7 @@ ResNet-50 data-parallel training in bf16 at 1/2/4/8 B200.
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
       --master-port P bench.py --gpus N --steps K --warmup W           # N > 1
   python bench.py --impl reference ...                                 # the UNMODIFIED reference from baseline/_ref
+  python bench.py ... --dump-outputs DIR                               # + the last timed step's loss and parameters as .npy
 
 Workload (identical in both arms; weak scaling - per-GPU work fixed):
   ResNet-50, random init, bf16 compute; per-GPU batch 32 (the reference's --per_gpu_train_batch_size default,
@@ -68,7 +69,14 @@ def parse_args():
     p.add_argument("--trace_dir", type=str, default=None, help="after the timed loops: 4 more steps under the CUPTI profiler, one chrome trace per rank "
                                                                   "(<dir>/rank<r>.json) for tools/trace_digest.py; never a timing source")
     p.add_argument("--no_broadcast_buffers", action="store_true", help="diagnostic: DDP without the per-step buffer broadcast")
+    p.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                   help="--impl ours: after the timed loops, write what the last timed step left for its caller (the loss it returned "
+                        "and the updated parameters) as DIR/loss.npy and DIR/params.npy, so two builds can be compared output for output")
     args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs is only implemented for --impl ours")
     if args.per_gpu_batch is None:
         args.per_gpu_batch = 16 if args.model.startswith("bert") else 32
     return args
@@ -168,6 +176,26 @@ def opt_ins(model):
         if os.environ.get(key):
             out[key] = os.environ[key]
     return {"opt_in": out} if out else {}
+
+
+DUMP_SAMPLE = 1 << 22      # elements kept per array (16 MB): positions drawn from a fixed seed, the same in every build
+
+
+def dump_outputs(out_dir, loss, model):
+    """What the caller of a training step holds after it, as float32 arrays: the loss the step returned (loss.npy) and
+    the parameters it updated, flattened and concatenated in module order (params.npy), reduced to a seeded sample of
+    DUMP_SAMPLE elements when longer.  Gradients and BatchNorm running statistics are not written: on a randomly
+    initialised bf16 ResNet two runs of the same build already disagree on them (the gradients below the head
+    entirely, the last stage's running statistics by a few percent), so they cannot tell two builds apart."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, tensors in (("loss", [loss]), ("params", list(model.parameters()))):
+        flat = torch.cat([t.detach().reshape(-1).float() for t in tensors])
+        if flat.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), flat.cpu().numpy())
 
 
 def config_dict(args, world, extra=None):
@@ -300,7 +328,7 @@ def run_ours(args):
     ev0.record()
     for i in range(args.steps):
         x, y = resident[i % len(resident)]
-        step(x, y)
+        loss = step(x, y)
         sched.step()
     ev1.record()
     sync_all()
@@ -337,6 +365,8 @@ def run_ours(args):
         last_loss = float(loss_ring[(args.steps - 1) % len(loss_ring)])
         e2e = {"ms": ms_e2e, "h2d": h2d_bytes / args.steps, "d2h": d2h_bytes / args.steps, "last_loss": last_loss,
                "loader_wait_ms": wait_s * 1e3 / args.steps}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, inner)         # `loss`: what the last timed step returned
 
     # ---- reduce over ranks (max time) ---------------------------------------------------------------
     def max_over_ranks(v):

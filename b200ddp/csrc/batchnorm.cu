@@ -18,8 +18,6 @@
 // channel tile finishes the reduction in a fixed order (no float atomics -> bitwise reproducible).
 #include "ops.h"
 
-#include <cstdlib>
-
 namespace b200 {
 namespace {
 
@@ -50,6 +48,27 @@ struct Tile {
   int grid_y;    // row splits
 };
 
+// Where a thread works in every kernel below: column tx of its block's cvb channel vectors (global channel vector cv, i.e.
+// channels cv*8 .. cv*8+7) and row lane tyi of ty.
+struct BnThread {
+  int tx, tyi, cv;
+};
+__device__ __forceinline__ BnThread bn_thread(int cvb) {
+  BnThread t;
+  t.tx = threadIdx.x % cvb;
+  t.tyi = threadIdx.x / cvb;
+  t.cv = blockIdx.x * cvb + t.tx;
+  return t;
+}
+
+// Rows [x, y) of R: this block's share of the gridDim.y row splits.
+__device__ __forceinline__ int2 bn_row_split(int R) {
+  const int S = gridDim.y;
+  const int rows_per = (R + S - 1) / S;
+  const int r0 = blockIdx.y * rows_per;
+  return make_int2(r0, min(R, r0 + rows_per));
+}
+
 // Block-level reduction over the `ty` row-lanes of two 8-wide accumulators; result valid for threads with row-lane 0.
 template <int NACC>
 __device__ __forceinline__ void reduce_rows(float (*acc)[kVec], float* smem, int tx, int tyi, int cvb, int ty) {
@@ -69,58 +88,89 @@ __device__ __forceinline__ void reduce_rows(float (*acc)[kVec], float* smem, int
   __syncthreads();
 }
 
+// Finishes a two-sum column reduction across the gridDim.y row splits of a channel tile, deterministically (no float atomics).
+// Every block publishes its totals, left in smem by reduce_rows<2>, to partial = [2][S][C] and takes a ticket on its tile's
+// counter.  The last block to arrive sums the S partials in a fixed order and calls epilogue(ch, s, q, 1/R) once per channel
+// of the tile.  Returns true in that block only; after a __syncthreads it must reset counters[blockIdx.x] to 0 for the next
+// launch (graph replay safe).
+template <typename Epilogue>
+__device__ __forceinline__ bool bn_finish_tile(float* __restrict__ partial, unsigned int* __restrict__ counters, float* smem, int R, int C,
+                                               int cvb, int ty, Epilogue epilogue) {
+  __shared__ bool is_last;
+  const int S = gridDim.y;
+  const int width = cvb * kVec;
+  const int c0 = blockIdx.x * width;
+  for (int c = threadIdx.x; c < width; c += blockDim.x) {
+    if (c0 + c < C) {
+      partial[(size_t)(0 * S + blockIdx.y) * C + c0 + c] = smem[c];
+      partial[(size_t)(1 * S + blockIdx.y) * C + c0 + c] = smem[ty * width + c];
+    }
+  }
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const unsigned int ticket = atomicAdd(&counters[blockIdx.x], 1u);
+    is_last = (ticket == (unsigned int)S - 1);
+  }
+  __syncthreads();
+  if (!is_last) return false;
+  __threadfence();
+  const float inv_r = 1.f / (float)R;
+  // `lanes` threads per channel each sum a strided subset of the S partials (independent loads in flight),
+  // then a fixed-order combine through shared memory
+  const int lanes = max(1, (int)blockDim.x / width);
+  {
+    const int c = threadIdx.x % width, l = threadIdx.x / width;
+    float ps = 0.f, pq = 0.f;
+    if (l < lanes && c0 + c < C) {
+#pragma unroll 4
+      for (int k = l; k < S; k += lanes) { ps += __ldcg(&partial[(size_t)(0 * S + k) * C + c0 + c]); pq += __ldcg(&partial[(size_t)(1 * S + k) * C + c0 + c]); }
+    }
+    __syncthreads();
+    if (l < lanes) { smem[l * width + c] = ps; smem[(lanes + l) * width + c] = pq; }
+    __syncthreads();
+  }
+  for (int c = threadIdx.x; c < width; c += blockDim.x) {
+    const int ch = c0 + c;
+    if (ch >= C) continue;
+    float s = 0.f, q = 0.f;
+    for (int l = 0; l < lanes; ++l) { s += smem[l * width + c]; q += smem[(lanes + l) * width + c]; }
+    epilogue(ch, s, q, inv_r);
+  }
+  return true;
+}
+
+// Block totals of this thread's 8 channels over the G rows of partial = [2][G][C] (rows strided over the row lanes, then
+// reduce_rows<2>): the first sums land at smem[tx*8 + i], the second at smem[ty*width + tx*8 + i].
+__device__ __forceinline__ void bn_reduce_partials(const float* __restrict__ partial, int G, int C, bool live, int cv, int tx, int tyi, int cvb,
+                                                   int ty, float* smem) {
+  float acc[2][kVec];
+#pragma unroll
+  for (int i = 0; i < kVec; ++i) { acc[0][i] = 0.f; acc[1][i] = 0.f; }
+  if (live) {
+    for (int g = tyi; g < G; g += ty) {
+      float a[kVec], b[kVec];
+      bn_load8<float>(partial + (size_t)g * C + cv * kVec, a);
+      bn_load8<float>(partial + ((size_t)G + g) * C + cv * kVec, b);
+#pragma unroll
+      for (int i = 0; i < kVec; ++i) { acc[0][i] += a[i]; acc[1][i] += b[i]; }
+    }
+  }
+  reduce_rows<2>(acc, smem, tx, tyi, cvb, ty);
+}
+
 // ------------------------------------------------------------------------------------------------------
 template <typename T>
-__device__ __forceinline__ void bn_apply_rows(const T* __restrict__ x, const T* __restrict__ residual, T* __restrict__ y,
-                                              unsigned char* __restrict__ mask, const float* __restrict__ scale,
-                                              const float* __restrict__ shift, int C, int cv, int r0, int r1, int tyi, int ty, int relu);
-
-// Programmatic dependent launch (opt-in, B200DDP_PDL=1): the producer lets the dependent grid start scheduling once its
-// main loop is done; the dependent blocks at griddepcontrol.wait until the producer grid has completed and flushed.
-__device__ __forceinline__ void bn_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void bn_wait_producer() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-// release/acquire on the per-tile generation word used by the fused (single-launch) variants
-__device__ __forceinline__ void bn_st_release(unsigned int* p, unsigned int v) { asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-__device__ __forceinline__ unsigned int bn_ld_acquire(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-// bounded spin (2 s): a scheduling surprise must degrade into a wrong number, never into a hung GPU
-__device__ __forceinline__ void bn_wait_generation(const unsigned int* p, unsigned int gen0) {
-  unsigned long long t0;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-  while (bn_ld_acquire(p) == gen0) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    if (t - t0 > 2000000000ull) break;
-  }
-}
-
-// FUSED = true: statistics AND normalisation in ONE launch.  All blocks of a channel tile rendezvous on a
-// generation word after the tile's last block has finished the statistics (the grid is sized to be co-resident:
-// <= 2 blocks per SM), then every block normalises exactly the rows it has just read (L2-hot).
-template <typename T, bool FUSED, bool PDL = false>
 __global__ void __launch_bounds__(kBnThreads, 2) bn_stats_kernel(const T* __restrict__ x, int R, int C, int cvb, int ty,
                                                              float* __restrict__ partial /*[2][S][C]*/, unsigned int* __restrict__ counters,
                                                              const float* __restrict__ gamma, const float* __restrict__ beta,
                                                              float* __restrict__ running_mean, float* __restrict__ running_var,
                                                              long long* __restrict__ num_batches, float* __restrict__ save_mean,
                                                              float* __restrict__ save_rstd, float* __restrict__ scale, float* __restrict__ shift,
-                                                             float eps, float momentum, const T* __restrict__ residual, T* __restrict__ y,
-                                                             unsigned char* __restrict__ mask, int relu) {
+                                                             float eps, float momentum) {
   extern __shared__ float smem[];
-  __shared__ bool is_last;
-  unsigned int* gen = counters + gridDim.x;             // [grid_x] generation words behind the [grid_x] ticket counters
-  unsigned int gen0 = 0;
-  if (FUSED && threadIdx.x == 0) gen0 = *reinterpret_cast<volatile unsigned int*>(&gen[blockIdx.x]);   // read BEFORE taking a ticket
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;                 // channel-vector index
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
+  const auto [tx, tyi, cv] = bn_thread(cvb);
+  const auto [r0, r1] = bn_row_split(R);
   float acc[2][kVec];
 #pragma unroll
   for (int i = 0; i < kVec; ++i) { acc[0][i] = 0.f; acc[1][i] = 0.f; }
@@ -143,72 +193,28 @@ __global__ void __launch_bounds__(kBnThreads, 2) bn_stats_kernel(const T* __rest
       for (int i = 0; i < kVec; ++i) { acc[0][i] += f[i]; acc[1][i] = fmaf(f[i], f[i], acc[1][i]); }
     }
   }
-  if constexpr (PDL) bn_launch_dependents();       // the apply kernel may start scheduling; it still waits for this whole grid
   reduce_rows<2>(acc, smem, tx, tyi, cvb, ty);
-  const int width = cvb * kVec;
-  const int c0 = blockIdx.x * width;
-  for (int c = threadIdx.x; c < width; c += blockDim.x) {
-    if (c0 + c < C) {
-      partial[(size_t)(0 * S + blockIdx.y) * C + c0 + c] = smem[c];
-      partial[(size_t)(1 * S + blockIdx.y) * C + c0 + c] = smem[ty * width + c];
+  const auto epilogue = [&](int ch, float s, float q, float inv_r) {
+    const float mean = s * inv_r;
+    const float var = fmaxf(q * inv_r - mean * mean, 0.f);     // biased variance (normalisation)
+    const float rstd = rsqrtf(var + eps);
+    const float sc = gamma[ch] * rstd;
+    save_mean[ch] = mean;
+    save_rstd[ch] = rstd;
+    scale[ch] = sc;
+    shift[ch] = beta[ch] - mean * sc;
+    if (running_mean != nullptr) {
+      const float unbiased = R > 1 ? var * ((float)R / (float)(R - 1)) : var;
+      running_mean[ch] = (1.f - momentum) * running_mean[ch] + momentum * mean;
+      running_var[ch] = (1.f - momentum) * running_var[ch] + momentum * unbiased;
     }
-  }
-  __threadfence();
+  };
+  if (!bn_finish_tile(partial, counters, smem, R, C, cvb, ty, epilogue)) return;
   __syncthreads();
   if (threadIdx.x == 0) {
-    const unsigned int ticket = atomicAdd(&counters[blockIdx.x], 1u);
-    is_last = (ticket == (unsigned int)S - 1);
+    counters[blockIdx.x] = 0u;                                 // ready for the next launch (graph replay safe)
+    if (blockIdx.x == 0 && num_batches != nullptr) *num_batches += 1;
   }
-  __syncthreads();
-  if (!FUSED && !is_last) return;
-  if (is_last) {
-    __threadfence();
-    const float inv_r = 1.f / (float)R;
-    // finish: `lanes` threads per channel each sum a strided subset of the S partials (independent loads in flight),
-    // then a fixed-order combine through shared memory
-    const int lanes = max(1, (int)blockDim.x / width);
-    {
-      const int c = threadIdx.x % width, l = threadIdx.x / width;
-      float ps = 0.f, pq = 0.f;
-      if (l < lanes && c0 + c < C) {
-  #pragma unroll 4
-        for (int k = l; k < S; k += lanes) { ps += __ldcg(&partial[(size_t)(0 * S + k) * C + c0 + c]); pq += __ldcg(&partial[(size_t)(1 * S + k) * C + c0 + c]); }
-      }
-      __syncthreads();
-      if (l < lanes) { smem[l * width + c] = ps; smem[(lanes + l) * width + c] = pq; }
-      __syncthreads();
-    }
-    for (int c = threadIdx.x; c < width; c += blockDim.x) {
-      const int ch = c0 + c;
-      if (ch >= C) continue;
-      float s = 0.f, q = 0.f;
-      for (int l = 0; l < lanes; ++l) { s += smem[l * width + c]; q += smem[(lanes + l) * width + c]; }
-      const float mean = s * inv_r;
-      const float var = fmaxf(q * inv_r - mean * mean, 0.f);     // biased variance (normalisation)
-      const float rstd = rsqrtf(var + eps);
-      const float sc = gamma[ch] * rstd;
-      save_mean[ch] = mean;
-      save_rstd[ch] = rstd;
-      scale[ch] = sc;
-      shift[ch] = beta[ch] - mean * sc;
-      if (running_mean != nullptr) {
-        const float unbiased = R > 1 ? var * ((float)R / (float)(R - 1)) : var;
-        running_mean[ch] = (1.f - momentum) * running_mean[ch] + momentum * mean;
-        running_var[ch] = (1.f - momentum) * running_var[ch] + momentum * unbiased;
-      }
-    }
-
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      counters[blockIdx.x] = 0u;                                 // ready for the next launch (graph replay safe)
-      if (blockIdx.x == 0 && num_batches != nullptr) *num_batches += 1;
-      if (FUSED) { __threadfence(); bn_st_release(&gen[blockIdx.x], gen0 + 1u); }
-    }
-  }
-  if (!FUSED) return;
-  if (!is_last && threadIdx.x == 0) bn_wait_generation(&gen[blockIdx.x], gen0);      // the tile's statistics are final
-  __syncthreads();
-  if (cv * kVec < C) bn_apply_rows<T>(x, residual, y, mask, scale, shift, C, cv, r0, r1, tyi, ty, relu);
 }
 
 template <typename T>
@@ -262,59 +268,22 @@ template <typename T>
 __global__ void __launch_bounds__(kBnThreads) bn_apply_kernel(const T* __restrict__ x, const T* __restrict__ residual, T* __restrict__ y,
                                                              unsigned char* __restrict__ mask, const float* __restrict__ scale,
                                                              const float* __restrict__ shift, int R, int C, int cvb, int ty, int relu) {
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;
+  const auto [tx, tyi, cv] = bn_thread(cvb);
   if (cv * kVec >= C) return;
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
+  const auto [r0, r1] = bn_row_split(R);
   bn_apply_rows<T>(x, residual, y, mask, scale, shift, C, cv, r0, r1, tyi, ty, relu);
 }
-
-// same body, launched as a programmatic dependent of bn_stats_kernel<.., PDL = true>
-template <typename T>
-__global__ void __launch_bounds__(kBnThreads) bn_apply_pdl_kernel(const T* __restrict__ x, const T* __restrict__ residual, T* __restrict__ y,
-                                                                 unsigned char* __restrict__ mask, const float* __restrict__ scale,
-                                                                 const float* __restrict__ shift, int R, int C, int cvb, int ty, int relu) {
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
-  bn_wait_producer();                               // scale / shift are written by the producer's last block
-  if (cv * kVec >= C) return;
-  bn_apply_rows<T>(x, residual, y, mask, scale, shift, C, cv, r0, r1, tyi, ty, relu);
-}
-
-template <typename T>
-__device__ __forceinline__ void bn_bwd_apply_rows(const T* __restrict__ dy, const T* __restrict__ x, const unsigned char* __restrict__ y,
-                                                  T* __restrict__ dx, T* __restrict__ dres, const float* __restrict__ save_mean,
-                                                  const float* __restrict__ save_rstd, const float* __restrict__ gamma,
-                                                  const float* __restrict__ coef, int C, int cv, int r0, int r1, int tyi, int ty, int relu);
-template <typename T>
-__device__ __forceinline__ void bn_bwd_apply_rows_coef(const T* __restrict__ dy, const T* __restrict__ x, const unsigned char* __restrict__ y,
-                                                       T* __restrict__ dx, T* __restrict__ dres, const float* __restrict__ save_mean,
-                                                       const float* __restrict__ save_rstd, const float* __restrict__ gamma,
-                                                       const float* c1p, const float* c2p, int C, int cv, int r0, int r1, int tyi, int ty, int relu);
 
 // ------------------------------------------------------------------------------------------------------
-template <typename T, bool FUSED, bool PDL = false>
+template <typename T>
 __global__ void __launch_bounds__(kBnThreads, 2) bn_bwd_reduce_kernel(const T* __restrict__ dy, const T* __restrict__ x, const unsigned char* __restrict__ y,
                                                                      int R, int C, int cvb, int ty, int relu, const float* __restrict__ save_mean,
                                                                      const float* __restrict__ save_rstd, float* __restrict__ partial,
                                                                      unsigned int* __restrict__ counters, float* __restrict__ dgamma,
-                                                                     float* __restrict__ dbeta, float* __restrict__ coef /*[2][C]*/,
-                                                                     const float* __restrict__ gamma, T* __restrict__ dx, T* __restrict__ dres) {
+                                                                     float* __restrict__ dbeta, float* __restrict__ coef /*[2][C]*/) {
   extern __shared__ float smem[];
-  __shared__ bool is_last;
-  unsigned int* gen = counters + gridDim.x;
-  unsigned int gen0 = 0;
-  if (FUSED && threadIdx.x == 0) gen0 = *reinterpret_cast<volatile unsigned int*>(&gen[blockIdx.x]);
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
+  const auto [tx, tyi, cv] = bn_thread(cvb);
+  const auto [r0, r1] = bn_row_split(R);
   float acc[2][kVec];
 #pragma unroll
   for (int i = 0; i < kVec; ++i) { acc[0][i] = 0.f; acc[1][i] = 0.f; }
@@ -357,62 +326,16 @@ __global__ void __launch_bounds__(kBnThreads, 2) bn_bwd_reduce_kernel(const T* _
       }
     }
   }
-  if constexpr (PDL) bn_launch_dependents();       // the apply kernel may start scheduling; it still waits for this whole grid
   reduce_rows<2>(acc, smem, tx, tyi, cvb, ty);
-  const int width = cvb * kVec;
-  const int c0 = blockIdx.x * width;
-  for (int c = threadIdx.x; c < width; c += blockDim.x) {
-    if (c0 + c < C) {
-      partial[(size_t)(0 * S + blockIdx.y) * C + c0 + c] = smem[c];
-      partial[(size_t)(1 * S + blockIdx.y) * C + c0 + c] = smem[ty * width + c];
-    }
-  }
-  __threadfence();
+  const auto epilogue = [&](int ch, float s, float q, float inv_r) {
+    dbeta[ch] = s;
+    dgamma[ch] = q;
+    coef[ch] = s * inv_r;            // mean(dy*)
+    coef[C + ch] = q * inv_r;        // mean(dy* xhat)
+  };
+  if (!bn_finish_tile(partial, counters, smem, R, C, cvb, ty, epilogue)) return;
   __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int ticket = atomicAdd(&counters[blockIdx.x], 1u);
-    is_last = (ticket == (unsigned int)S - 1);
-  }
-  __syncthreads();
-  if (!FUSED && !is_last) return;
-  if (is_last) {
-    __threadfence();
-    const float inv_r = 1.f / (float)R;
-    // finish: `lanes` threads per channel each sum a strided subset of the S partials (independent loads in flight),
-    // then a fixed-order combine through shared memory
-    const int lanes = max(1, (int)blockDim.x / width);
-    {
-      const int c = threadIdx.x % width, l = threadIdx.x / width;
-      float ps = 0.f, pq = 0.f;
-      if (l < lanes && c0 + c < C) {
-  #pragma unroll 4
-        for (int k = l; k < S; k += lanes) { ps += __ldcg(&partial[(size_t)(0 * S + k) * C + c0 + c]); pq += __ldcg(&partial[(size_t)(1 * S + k) * C + c0 + c]); }
-      }
-      __syncthreads();
-      if (l < lanes) { smem[l * width + c] = ps; smem[(lanes + l) * width + c] = pq; }
-      __syncthreads();
-    }
-    for (int c = threadIdx.x; c < width; c += blockDim.x) {
-      const int ch = c0 + c;
-      if (ch >= C) continue;
-      float s = 0.f, q = 0.f;
-      for (int l = 0; l < lanes; ++l) { s += smem[l * width + c]; q += smem[(lanes + l) * width + c]; }
-      dbeta[ch] = s;
-      dgamma[ch] = q;
-      coef[ch] = s * inv_r;            // mean(dy*)
-      coef[C + ch] = q * inv_r;        // mean(dy* xhat)
-    }
-
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      counters[blockIdx.x] = 0u;
-      if (FUSED) { __threadfence(); bn_st_release(&gen[blockIdx.x], gen0 + 1u); }
-    }
-  }
-  if (!FUSED) return;
-  if (!is_last && threadIdx.x == 0) bn_wait_generation(&gen[blockIdx.x], gen0);
-  __syncthreads();
-  if (cv * kVec < C) bn_bwd_apply_rows<T>(dy, x, y, dx, dres, save_mean, save_rstd, gamma, coef, C, cv, r0, r1, tyi, ty, relu);
+  if (threadIdx.x == 0) counters[blockIdx.x] = 0u;
 }
 
 // c1p / c2p point at THIS thread's 8 coefficients (global coef rows or a block's shared-memory copy)
@@ -479,62 +402,14 @@ __device__ __forceinline__ void bn_bwd_apply_rows_coef(const T* __restrict__ dy,
 }
 
 template <typename T>
-__device__ __forceinline__ void bn_bwd_apply_rows(const T* __restrict__ dy, const T* __restrict__ x, const unsigned char* __restrict__ y,
-                                                  T* __restrict__ dx, T* __restrict__ dres, const float* __restrict__ save_mean,
-                                                  const float* __restrict__ save_rstd, const float* __restrict__ gamma,
-                                                  const float* __restrict__ coef, int C, int cv, int r0, int r1, int tyi, int ty, int relu) {
-  bn_bwd_apply_rows_coef<T>(dy, x, y, dx, dres, save_mean, save_rstd, gamma, coef + cv * kVec, coef + C + cv * kVec, C, cv, r0, r1, tyi, ty, relu);
-}
-
-template <typename T>
 __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_kernel(const T* __restrict__ dy, const T* __restrict__ x, const unsigned char* __restrict__ y,
                                                                  T* __restrict__ dx, T* __restrict__ dres, const float* __restrict__ save_mean,
                                                                  const float* __restrict__ save_rstd, const float* __restrict__ gamma,
                                                                  const float* __restrict__ coef, int R, int C, int cvb, int ty, int relu) {
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;
+  const auto [tx, tyi, cv] = bn_thread(cvb);
   if (cv * kVec >= C) return;
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
-  bn_bwd_apply_rows<T>(dy, x, y, dx, dres, save_mean, save_rstd, gamma, coef, C, cv, r0, r1, tyi, ty, relu);
-}
-
-template <typename T>
-__global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_pdl_kernel(const T* __restrict__ dy, const T* __restrict__ x, const unsigned char* __restrict__ y,
-                                                                     T* __restrict__ dx, T* __restrict__ dres, const float* __restrict__ save_mean,
-                                                                     const float* __restrict__ save_rstd, const float* __restrict__ gamma,
-                                                                     const float* __restrict__ coef, int R, int C, int cvb, int ty, int relu) {
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
-  bn_wait_producer();                               // coef / dgamma / dbeta come from the producer's last block
-  if (cv * kVec >= C) return;
-  bn_bwd_apply_rows<T>(dy, x, y, dx, dres, save_mean, save_rstd, gamma, coef, C, cv, r0, r1, tyi, ty, relu);
-}
-
-// B200DDP_PDL=1: stats -> apply and bwd_reduce -> bwd_apply become programmatic dependent launches
-int g_bn_pdl = -1;     // -1: read B200DDP_PDL on first use
-bool bn_pdl_enabled() {
-  if (g_bn_pdl < 0) { const char* e = getenv("B200DDP_PDL"); g_bn_pdl = (e && atoi(e) != 0) ? 1 : 0; }
-  return g_bn_pdl > 0;
-}
-
-template <typename... KArgs, typename... Args>
-void launch_dependent(void (*kernel)(KArgs...), dim3 grid, cudaStream_t s, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(kBnThreads);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  B200_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...));
+  const auto [r0, r1] = bn_row_split(R);
+  bn_bwd_apply_rows_coef<T>(dy, x, y, dx, dres, save_mean, save_rstd, gamma, coef + cv * kVec, coef + C + cv * kVec, C, cv, r0, r1, tyi, ty, relu);
 }
 
 Tile pick_tile(int R, int C) {
@@ -562,18 +437,11 @@ dim3 apply_grid(const Tile& t, int R) {
   return dim3(t.grid_x, gy);
 }
 
-// Fused (single-launch) variants need every block of a channel tile resident at once: cap the grid at 2 blocks per SM.
-bool fused_tile(int R, int C, Tile* t) {
-  static int enabled = -1;
-  // measured (profiles/README.md): one launch per direction is NOT faster than two at batch 32 (the co-residency cap
-  // on the grid costs what the saved launch gains), so the two-launch form stays the default; opt in with =1
-  if (enabled < 0) { const char* e = getenv("B200DDP_BN_FUSED"); enabled = (e && atoi(e) == 1) ? 1 : 0; }
-  *t = pick_tile(R, C);
-  if (!enabled || t->grid_x > 2 * kNumSMs) return false;
-  int cap = (2 * kNumSMs) / t->grid_x;
-  if (cap < 1) cap = 1;
-  if (t->grid_y > cap) t->grid_y = cap;
-  return true;
+// Calls launch(T()) with T the element type of `dt`: bf16, anything else fp32.
+template <typename Launch>
+void with_element_type(DType dt, Launch&& launch) {
+  if (dt == DType::BF16) launch(__nv_bfloat16());
+  else launch(float());
 }
 
 }  // namespace
@@ -592,22 +460,9 @@ __global__ void __launch_bounds__(kBnThreads) bn_apply_partials_kernel(const T* 
                                                                       float* __restrict__ save_rstd, float eps, float momentum, int R, int C,
                                                                       int cvb, int ty, int relu) {
   extern __shared__ float bn_smem[];                 // [2][ty][cvb*8] reduction scratch, then [2][cvb*8] scale / shift
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;
+  const auto [tx, tyi, cv] = bn_thread(cvb);
   const bool live = cv * kVec < C;
-  float acc[2][kVec];
-#pragma unroll
-  for (int i = 0; i < kVec; ++i) { acc[0][i] = 0.f; acc[1][i] = 0.f; }
-  if (live) {
-    for (int g = tyi; g < G; g += ty) {
-      float a[kVec], b[kVec];
-      bn_load8<float>(partial + (size_t)g * C + cv * kVec, a);
-      bn_load8<float>(partial + ((size_t)G + g) * C + cv * kVec, b);
-#pragma unroll
-      for (int i = 0; i < kVec; ++i) { acc[0][i] += a[i]; acc[1][i] += b[i]; }
-    }
-  }
-  reduce_rows<2>(acc, bn_smem, tx, tyi, cvb, ty);
+  bn_reduce_partials(partial, G, C, live, cv, tx, tyi, cvb, ty, bn_smem);
   const int width = cvb * kVec;
   float* sc_s = bn_smem + 2 * ty * width;            // scale / shift of this block's channels
   float* sh_s = sc_s + width;
@@ -637,9 +492,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_apply_partials_kernel(const T* 
   if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0 && num_batches != nullptr) *num_batches += 1;
   __syncthreads();
   if (!live) return;
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
+  const auto [r0, r1] = bn_row_split(R);
   // bn_apply_rows indexes scale / shift by the global channel vector: hand it pointers rebased to this block's tile
   bn_apply_rows<T>(x, residual, y, mask, sc_s - (size_t)blockIdx.x * width, sh_s - (size_t)blockIdx.x * width, C, cv, r0, r1, tyi, ty, relu);
 }
@@ -654,24 +507,11 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_partials_kernel(const
                                                                           const float* __restrict__ gamma, float* __restrict__ dgamma,
                                                                           float* __restrict__ dbeta, int R, int C, int cvb, int ty, int relu) {
   extern __shared__ float bn_smem[];                 // [2][ty][cvb*8] reduction scratch, then [2][cvb*8] coefficients
-  const int tx = threadIdx.x % cvb, tyi = threadIdx.x / cvb;
-  const int cv = blockIdx.x * cvb + tx;
+  const auto [tx, tyi, cv] = bn_thread(cvb);
   const bool live = cv * kVec < C;
-  float acc[2][kVec];
-#pragma unroll
-  for (int i = 0; i < kVec; ++i) { acc[0][i] = 0.f; acc[1][i] = 0.f; }
-  if (live) {
-    for (int g = tyi; g < G; g += ty) {
-      float a[kVec], b[kVec];
-      bn_load8<float>(partial + (size_t)g * C + cv * kVec, a);
-      bn_load8<float>(partial + ((size_t)G + g) * C + cv * kVec, b);
-#pragma unroll
-      for (int i = 0; i < kVec; ++i) { acc[0][i] += a[i]; acc[1][i] += b[i]; }
-    }
-  }
-  reduce_rows<2>(acc, bn_smem, tx, tyi, cvb, ty);
+  bn_reduce_partials(partial, G, C, live, cv, tx, tyi, cvb, ty, bn_smem);
   const int width = cvb * kVec;
-  float* c1_s = bn_smem + 2 * ty * width;            // coef layout expected by bn_bwd_apply_rows: c1 at [0, C), c2 at [C, 2C)
+  float* c1_s = bn_smem + 2 * ty * width;            // c1 / c2 of this block's channels
   float* c2_s = c1_s + width;
   if (tyi == 0 && live) {
     const float inv_r = 1.f / (float)R;
@@ -686,21 +526,14 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_partials_kernel(const
   }
   __syncthreads();
   if (!live) return;
-  const int S = gridDim.y;
-  const int rows_per = (R + S - 1) / S;
-  const int r0 = blockIdx.y * rows_per, r1 = min(R, r0 + rows_per);
-  // bn_bwd_apply_rows reads coef[cv*8 + i] and coef[C + cv*8 + i]: rebase so that both land in this block's two smem rows
-  // (c2 row sits `width` floats after c1: a fake "C" of `width` would break the global indexing of the other operands, so the
-  // coefficients are passed through a two-pointer variant)
+  const auto [r0, r1] = bn_row_split(R);
   bn_bwd_apply_rows_coef<T>(dy, x, y, dx, dres, save_mean, save_rstd, gamma, c1_s + tx * kVec, c2_s + tx * kVec, C, cv, r0, r1, tyi, ty, relu);
 }
-
-void set_bn_pdl(int on) { g_bn_pdl = on; }
 
 void bn_workspace_sizes(int R, int C, size_t* partial_floats, size_t* counters) {
   const Tile t = pick_tile(R, C);
   *partial_floats = (size_t)2 * t.grid_y * C;
-  *counters = (size_t)2 * t.grid_x;          // tickets + generation words
+  *counters = (size_t)t.grid_x;              // one self-resetting ticket counter per channel tile
 }
 
 void launch_bn_forward(const void* x, const void* residual, void* y, unsigned char* mask, DType dt, int R, int C, const float* gamma, const float* beta,
@@ -708,62 +541,36 @@ void launch_bn_forward(const void* x, const void* residual, void* y, unsigned ch
                        float* scale, float* shift, float* partial, unsigned int* counters, float eps, float momentum, bool relu,
                        cudaStream_t s) {
   if (C % kVec != 0) throw std::runtime_error("fused batch norm: channel count must be a multiple of 8");
-  Tile t;
-  const bool fused = fused_tile(R, C, &t);
+  const Tile t = pick_tile(R, C);
   const size_t smem = (size_t)2 * t.ty * t.cvb * kVec * sizeof(float);
-  const dim3 grid(t.grid_x, t.grid_y);
   const int r = relu ? 1 : 0;
-  if (!fused && bn_pdl_enabled()) {
-    // opt-in: producer with an early launch_dependents, apply kernel as its programmatic dependent
-#define B200_BN_FWD_PDL(T)                                                                                                                  \
-    bn_stats_kernel<T, false, true><<<grid, kBnThreads, smem, s>>>((const T*)x, R, C, t.cvb, t.ty, partial, counters, gamma, beta, running_mean, \
-                                                                   running_var, num_batches, save_mean, save_rstd, scale, shift, eps, momentum,  \
-                                                                   (const T*)residual, (T*)y, mask, r);                                          \
-    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);                                                                                   \
-    launch_dependent(bn_apply_pdl_kernel<T>, apply_grid(t, R), s, (const T*)x, (const T*)residual, (T*)y, mask, (const float*)scale,              \
-                     (const float*)shift, R, C, t.cvb, t.ty, r);                                                                                  \
-    B200_COUNT_LAUNCH(1)
-    if (dt == DType::BF16) { B200_BN_FWD_PDL(__nv_bfloat16); } else { B200_BN_FWD_PDL(float); }
-#undef B200_BN_FWD_PDL
-    return;
-  }
-#define B200_BN_FWD(T, F)                                                                                                            \
-  bn_stats_kernel<T, F><<<grid, kBnThreads, smem, s>>>((const T*)x, R, C, t.cvb, t.ty, partial, counters, gamma, beta, running_mean, \
-                                                       running_var, num_batches, save_mean, save_rstd, scale, shift, eps, momentum, \
-                                                       (const T*)residual, (T*)y, mask, r)
-  if (dt == DType::BF16) { if (fused) B200_BN_FWD(__nv_bfloat16, true); else B200_BN_FWD(__nv_bfloat16, false); }
-  else { if (fused) B200_BN_FWD(float, true); else B200_BN_FWD(float, false); }
-#undef B200_BN_FWD
-  B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
-  if (fused) return;
-  if (dt == DType::BF16)
-    bn_apply_kernel<__nv_bfloat16><<<apply_grid(t, R), kBnThreads, 0, s>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)residual,
-                                                                           (__nv_bfloat16*)y, mask, scale, shift, R, C, t.cvb, t.ty, r);
-  else
-    bn_apply_kernel<float><<<apply_grid(t, R), kBnThreads, 0, s>>>((const float*)x, (const float*)residual, (float*)y, mask, scale, shift, R, C,
-                                                                   t.cvb, t.ty, r);
-  B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  with_element_type(dt, [&](auto elem) {
+    using T = decltype(elem);
+    bn_stats_kernel<T><<<dim3(t.grid_x, t.grid_y), kBnThreads, smem, s>>>((const T*)x, R, C, t.cvb, t.ty, partial, counters, gamma, beta,
+                                                                          running_mean, running_var, num_batches, save_mean, save_rstd,
+                                                                          scale, shift, eps, momentum);
+    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+    bn_apply_kernel<T><<<apply_grid(t, R), kBnThreads, 0, s>>>((const T*)x, (const T*)residual, (T*)y, mask, scale, shift, R, C, t.cvb, t.ty, r);
+    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  });
 }
 
 void launch_bn_forward_from_partials(const void* x, const void* residual, void* y, unsigned char* mask, DType dt, int R, int C,
                                      const float* gamma, const float* beta, float* running_mean, float* running_var,
-                                     long long* num_batches, float* save_mean, float* save_rstd, float* scale, float* shift,
-                                     const float* partial, int groups, float eps, float momentum, bool relu, cudaStream_t s) {
-  (void)scale; (void)shift;                          // each block derives them for its own channels (see bn_apply_partials_kernel)
+                                     long long* num_batches, float* save_mean, float* save_rstd, const float* partial, int groups,
+                                     float eps, float momentum, bool relu, cudaStream_t s) {
   if (C % kVec != 0) throw std::runtime_error("fused batch norm: channel count must be a multiple of 8");
   if (groups < 1) throw std::runtime_error("fused batch norm: empty partial statistics");
   const Tile t = pick_tile(R, C);
   const int r = relu ? 1 : 0;
   const size_t smem = (size_t)(2 * t.ty + 2) * t.cvb * kVec * sizeof(float);
-  if (dt == DType::BF16)
-    bn_apply_partials_kernel<__nv_bfloat16><<<apply_grid(t, R), kBnThreads, smem, s>>>(
-        (const __nv_bfloat16*)x, (const __nv_bfloat16*)residual, (__nv_bfloat16*)y, mask, partial, groups, gamma, beta, running_mean, running_var,
-        num_batches, save_mean, save_rstd, eps, momentum, R, C, t.cvb, t.ty, r);
-  else
-    bn_apply_partials_kernel<float><<<apply_grid(t, R), kBnThreads, smem, s>>>(
-        (const float*)x, (const float*)residual, (float*)y, mask, partial, groups, gamma, beta, running_mean, running_var, num_batches, save_mean,
-        save_rstd, eps, momentum, R, C, t.cvb, t.ty, r);
-  B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  with_element_type(dt, [&](auto elem) {
+    using T = decltype(elem);
+    bn_apply_partials_kernel<T><<<apply_grid(t, R), kBnThreads, smem, s>>>((const T*)x, (const T*)residual, (T*)y, mask, partial, groups, gamma,
+                                                                           beta, running_mean, running_var, num_batches, save_mean, save_rstd,
+                                                                           eps, momentum, R, C, t.cvb, t.ty, r);
+    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  });
 }
 
 void launch_bn_backward_from_partials(const void* dy, const void* x, const void* y, void* dx, void* dres, DType dt, int R, int C, const float* gamma,
@@ -774,56 +581,31 @@ void launch_bn_backward_from_partials(const void* dy, const void* x, const void*
   const Tile t = pick_tile(R, C);
   const int r = relu ? 1 : 0;
   const size_t smem = (size_t)(2 * t.ty + 2) * t.cvb * kVec * sizeof(float);
-  if (dt == DType::BF16)
-    bn_bwd_apply_partials_kernel<__nv_bfloat16><<<apply_grid(t, R), kBnThreads, smem, s>>>(
-        (const __nv_bfloat16*)dy, (const __nv_bfloat16*)x, (const unsigned char*)y, (__nv_bfloat16*)dx, (__nv_bfloat16*)dres, partial, groups, save_mean,
-        save_rstd, gamma, dgamma, dbeta, R, C, t.cvb, t.ty, r);
-  else
-    bn_bwd_apply_partials_kernel<float><<<apply_grid(t, R), kBnThreads, smem, s>>>(
-        (const float*)dy, (const float*)x, (const unsigned char*)y, (float*)dx, (float*)dres, partial, groups, save_mean, save_rstd, gamma, dgamma, dbeta,
-        R, C, t.cvb, t.ty, r);
-  B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  with_element_type(dt, [&](auto elem) {
+    using T = decltype(elem);
+    bn_bwd_apply_partials_kernel<T><<<apply_grid(t, R), kBnThreads, smem, s>>>((const T*)dy, (const T*)x, (const unsigned char*)y, (T*)dx, (T*)dres,
+                                                                               partial, groups, save_mean, save_rstd, gamma, dgamma, dbeta, R, C,
+                                                                               t.cvb, t.ty, r);
+    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  });
 }
 
 void launch_bn_backward(const void* dy, const void* x, const void* y, void* dx, void* dres, DType dt, int R, int C, const float* gamma,
                         const float* save_mean, const float* save_rstd, float* dgamma, float* dbeta, float* coef, float* partial,
                         unsigned int* counters, bool relu, cudaStream_t s) {
   if (C % kVec != 0) throw std::runtime_error("fused batch norm: channel count must be a multiple of 8");
-  Tile t;
-  const bool fused = fused_tile(R, C, &t);
+  const Tile t = pick_tile(R, C);
   const size_t smem = (size_t)2 * t.ty * t.cvb * kVec * sizeof(float);
-  const dim3 grid(t.grid_x, t.grid_y);
   const int r = relu ? 1 : 0;
-  if (!fused && bn_pdl_enabled()) {
-#define B200_BN_BWD_PDL(T)                                                                                                                    \
-    bn_bwd_reduce_kernel<T, false, true><<<grid, kBnThreads, smem, s>>>((const T*)dy, (const T*)x, (const unsigned char*)y, R, C, t.cvb, t.ty, r,  \
-                                                                        save_mean, save_rstd, partial, counters, dgamma, dbeta, coef, gamma,      \
-                                                                        (T*)dx, (T*)dres);                                                        \
-    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);                                                                                     \
-    launch_dependent(bn_bwd_apply_pdl_kernel<T>, apply_grid(t, R), s, (const T*)dy, (const T*)x, (const unsigned char*)y, (T*)dx, (T*)dres,         \
-                     save_mean, save_rstd, gamma, (const float*)coef, R, C, t.cvb, t.ty, r);                                                        \
-    B200_COUNT_LAUNCH(1)
-    if (dt == DType::BF16) { B200_BN_BWD_PDL(__nv_bfloat16); } else { B200_BN_BWD_PDL(float); }
-#undef B200_BN_BWD_PDL
-    return;
-  }
-#define B200_BN_BWD(T, F)                                                                                                              \
-  bn_bwd_reduce_kernel<T, F><<<grid, kBnThreads, smem, s>>>((const T*)dy, (const T*)x, (const unsigned char*)y, R, C, t.cvb, t.ty, r,  \
-                                                            save_mean, save_rstd, partial, counters, dgamma, dbeta, coef, gamma,      \
-                                                            (T*)dx, (T*)dres)
-  if (dt == DType::BF16) { if (fused) B200_BN_BWD(__nv_bfloat16, true); else B200_BN_BWD(__nv_bfloat16, false); }
-  else { if (fused) B200_BN_BWD(float, true); else B200_BN_BWD(float, false); }
-#undef B200_BN_BWD
-  B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
-  if (fused) return;
-  if (dt == DType::BF16)
-    bn_bwd_apply_kernel<__nv_bfloat16><<<apply_grid(t, R), kBnThreads, 0, s>>>((const __nv_bfloat16*)dy, (const __nv_bfloat16*)x, (const unsigned char*)y,
-                                                                               (__nv_bfloat16*)dx, (__nv_bfloat16*)dres, save_mean, save_rstd, gamma, coef,
-                                                                               R, C, t.cvb, t.ty, r);
-  else
-    bn_bwd_apply_kernel<float><<<apply_grid(t, R), kBnThreads, 0, s>>>((const float*)dy, (const float*)x, (const unsigned char*)y, (float*)dx,
-                                                                       (float*)dres, save_mean, save_rstd, gamma, coef, R, C, t.cvb, t.ty, r);
-  B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  with_element_type(dt, [&](auto elem) {
+    using T = decltype(elem);
+    bn_bwd_reduce_kernel<T><<<dim3(t.grid_x, t.grid_y), kBnThreads, smem, s>>>((const T*)dy, (const T*)x, (const unsigned char*)y, R, C, t.cvb, t.ty,
+                                                                               r, save_mean, save_rstd, partial, counters, dgamma, dbeta, coef);
+    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+    bn_bwd_apply_kernel<T><<<apply_grid(t, R), kBnThreads, 0, s>>>((const T*)dy, (const T*)x, (const unsigned char*)y, (T*)dx, (T*)dres, save_mean,
+                                                                   save_rstd, gamma, coef, R, C, t.cvb, t.ty, r);
+    B200_CUDA_CHECK(cudaGetLastError()); B200_COUNT_LAUNCH(1);
+  });
 }
 
 }  // namespace b200

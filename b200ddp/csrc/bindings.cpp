@@ -177,6 +177,57 @@ struct SgdPlan {
   }
 };
 
+// ---- fused BatchNorm: what the plain and the from-partials entry points share ------------------------------------------
+template <typename T>
+T* opt_ptr(const c10::optional<at::Tensor>& t) { return t.has_value() ? t->data_ptr<T>() : nullptr; }
+
+// Checked input x [N, C, H, W] channels_last (+ residual) and the outputs: y, stats = [4, C] (save_mean, save_rstd, scale,
+// shift) and, with relu, the [R, C/8] ReLU bitmask.
+struct BnForwardIo {
+  int R, C;
+  const void* res;
+  at::Tensor y, stats, mask;
+};
+BnForwardIo bn_forward_io(const char* op, const at::Tensor& x, const c10::optional<at::Tensor>& residual, const at::Tensor& gamma,
+                          const at::Tensor& beta, bool relu) {
+  check_cuda(x, "x");
+  TORCH_CHECK(x.dim() == 4 && x.is_contiguous(at::MemoryFormat::ChannelsLast), op, ": x must be 4-D channels_last");
+  TORCH_CHECK(gamma.scalar_type() == at::kFloat && beta.scalar_type() == at::kFloat, op, ": fp32 affine parameters");
+  BnForwardIo io;
+  io.C = (int)x.size(1);
+  io.R = (int)(x.numel() / io.C);
+  io.res = nullptr;
+  if (residual.has_value()) {
+    TORCH_CHECK(residual->sizes() == x.sizes() && residual->dtype() == x.dtype() && residual->is_contiguous(at::MemoryFormat::ChannelsLast),
+                op, ": residual must match x (shape, dtype, channels_last)");
+    io.res = residual->data_ptr();
+  }
+  io.y = at::empty_like(x);
+  io.stats = at::empty({4, io.C}, x.options().dtype(at::kFloat));
+  if (relu) io.mask = at::empty({(int64_t)io.R, (int64_t)(io.C / 8)}, x.options().dtype(at::kByte));
+  return io;
+}
+
+// Checked ReLU bitmask and the outputs: dx, dres (when asked for) and dparams = [rows, C] (dgamma, dbeta, then per-entry rows).
+struct BnBackwardIo {
+  int R, C;
+  const void* relu_mask;
+  at::Tensor dx, dres, dparams;
+};
+BnBackwardIo bn_backward_io(const char* op, const at::Tensor& dy, const at::Tensor& x, const c10::optional<at::Tensor>& y, bool relu,
+                            bool need_dres, int param_rows) {
+  check_cuda(dy, "dy");
+  TORCH_CHECK(!relu || (y.has_value() && y->scalar_type() == at::kByte), op, ": needs the ReLU bitmask written by bn_forward");
+  BnBackwardIo io;
+  io.C = (int)x.size(1);
+  io.R = (int)(x.numel() / io.C);
+  io.relu_mask = relu ? y->data_ptr() : nullptr;
+  io.dx = at::empty_like(x);
+  if (need_dres) io.dres = at::empty_like(x);
+  io.dparams = at::empty({param_rows, io.C}, x.options().dtype(at::kFloat));
+  return io;
+}
+
 }  // namespace
 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
@@ -662,7 +713,6 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   });
 
   // ---- fused BatchNorm ---------------------------------------------------------------------------
-  m.def("set_bn_pdl", &set_bn_pdl);
   m.def("bn_workspace", [](int R, int C) {
     size_t pf = 0, cn = 0;
     bn_workspace_sizes(R, C, &pf, &cn);
@@ -672,97 +722,57 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
                          c10::optional<at::Tensor> running_mean, c10::optional<at::Tensor> running_var,
                          c10::optional<at::Tensor> num_batches, double eps, double momentum, bool relu, at::Tensor partial,
                          at::Tensor counters) {
-    check_cuda(x, "x");
-    TORCH_CHECK(x.dim() == 4 && x.is_contiguous(at::MemoryFormat::ChannelsLast), "bn_forward: x must be 4-D channels_last");
-    TORCH_CHECK(gamma.scalar_type() == at::kFloat && beta.scalar_type() == at::kFloat, "bn_forward: fp32 affine parameters");
+    BnForwardIo io = bn_forward_io("bn_forward", x, residual, gamma, beta, relu);
     c10::cuda::CUDAGuard guard(x.device());
-    const int C = (int)x.size(1);
-    const int R = (int)(x.numel() / C);
-    at::Tensor y = at::empty_like(x);
-    auto fopt = x.options().dtype(at::kFloat);
-    at::Tensor stats = at::empty({4, C}, fopt);   // rows: save_mean, save_rstd, scale, shift
-    const void* res = nullptr;
-    if (residual.has_value()) {
-      TORCH_CHECK(residual->sizes() == x.sizes() && residual->dtype() == x.dtype() && residual->is_contiguous(at::MemoryFormat::ChannelsLast),
-                  "bn_forward: residual must match x (shape, dtype, channels_last)");
-      res = residual->data_ptr();
-    }
-    float* st = stats.data_ptr<float>();
-    at::Tensor mask = relu ? at::empty({(int64_t)R, (int64_t)(C / 8)}, x.options().dtype(at::kByte)) : at::Tensor();
-    launch_bn_forward(x.data_ptr(), res, y.data_ptr(), relu ? mask.data_ptr<uint8_t>() : nullptr, dtype_of(x), R, C, gamma.data_ptr<float>(), beta.data_ptr<float>(),
-                      running_mean.has_value() ? running_mean->data_ptr<float>() : nullptr,
-                      running_var.has_value() ? running_var->data_ptr<float>() : nullptr,
-                      num_batches.has_value() ? (long long*)num_batches->data_ptr<int64_t>() : nullptr, st, st + C, st + 2 * C, st + 3 * C,
-                      partial.data_ptr<float>(), (unsigned int*)counters.data_ptr<int>(), (float)eps, (float)momentum, relu, cur_stream());
-    return std::make_tuple(y, stats, mask);
+    float* st = io.stats.data_ptr<float>();
+    launch_bn_forward(x.data_ptr(), io.res, io.y.data_ptr(), relu ? io.mask.data_ptr<uint8_t>() : nullptr, dtype_of(x), io.R, io.C,
+                      gamma.data_ptr<float>(), beta.data_ptr<float>(), opt_ptr<float>(running_mean), opt_ptr<float>(running_var),
+                      (long long*)opt_ptr<int64_t>(num_batches), st, st + io.C, st + 2 * io.C, st + 3 * io.C, partial.data_ptr<float>(),
+                      (unsigned int*)counters.data_ptr<int>(), (float)eps, (float)momentum, relu, cur_stream());
+    return std::make_tuple(io.y, io.stats, io.mask);
   });
   m.def("bn_forward_partials", [](at::Tensor x, c10::optional<at::Tensor> residual, at::Tensor gamma, at::Tensor beta,
                                   c10::optional<at::Tensor> running_mean, c10::optional<at::Tensor> running_var,
                                   c10::optional<at::Tensor> num_batches, double eps, double momentum, bool relu, at::Tensor partial) {
-    check_cuda(x, "x"); check_cuda(partial, "partial");
-    TORCH_CHECK(x.dim() == 4 && x.is_contiguous(at::MemoryFormat::ChannelsLast), "bn_forward_partials: x must be 4-D channels_last");
-    TORCH_CHECK(gamma.scalar_type() == at::kFloat && beta.scalar_type() == at::kFloat, "bn_forward_partials: fp32 affine parameters");
-    const int C = (int)x.size(1);
-    const int R = (int)(x.numel() / C);
-    TORCH_CHECK(partial.scalar_type() == at::kFloat && partial.dim() == 3 && partial.size(0) == 2 && partial.size(2) == C &&
+    BnForwardIo io = bn_forward_io("bn_forward_partials", x, residual, gamma, beta, relu);
+    check_cuda(partial, "partial");
+    TORCH_CHECK(partial.scalar_type() == at::kFloat && partial.dim() == 3 && partial.size(0) == 2 && partial.size(2) == io.C &&
                 partial.is_contiguous(), "bn_forward_partials: partial statistics must be fp32 [2, groups, C]");
     c10::cuda::CUDAGuard guard(x.device());
-    at::Tensor y = at::empty_like(x);
-    at::Tensor stats = at::empty({4, C}, x.options().dtype(at::kFloat));   // rows: save_mean, save_rstd, scale, shift
-    const void* res = nullptr;
-    if (residual.has_value()) {
-      TORCH_CHECK(residual->sizes() == x.sizes() && residual->dtype() == x.dtype() && residual->is_contiguous(at::MemoryFormat::ChannelsLast),
-                  "bn_forward_partials: residual must match x (shape, dtype, channels_last)");
-      res = residual->data_ptr();
-    }
-    float* st = stats.data_ptr<float>();
-    at::Tensor mask = relu ? at::empty({(int64_t)R, (int64_t)(C / 8)}, x.options().dtype(at::kByte)) : at::Tensor();
-    launch_bn_forward_from_partials(x.data_ptr(), res, y.data_ptr(), relu ? mask.data_ptr<uint8_t>() : nullptr, dtype_of(x), R, C,
-                                    gamma.data_ptr<float>(), beta.data_ptr<float>(),
-                                    running_mean.has_value() ? running_mean->data_ptr<float>() : nullptr,
-                                    running_var.has_value() ? running_var->data_ptr<float>() : nullptr,
-                                    num_batches.has_value() ? (long long*)num_batches->data_ptr<int64_t>() : nullptr, st, st + C, st + 2 * C,
-                                    st + 3 * C, partial.data_ptr<float>(), (int)partial.size(1), (float)eps, (float)momentum, relu, cur_stream());
-    return std::make_tuple(y, stats, mask);
+    float* st = io.stats.data_ptr<float>();
+    launch_bn_forward_from_partials(x.data_ptr(), io.res, io.y.data_ptr(), relu ? io.mask.data_ptr<uint8_t>() : nullptr, dtype_of(x), io.R,
+                                    io.C, gamma.data_ptr<float>(), beta.data_ptr<float>(), opt_ptr<float>(running_mean),
+                                    opt_ptr<float>(running_var), (long long*)opt_ptr<int64_t>(num_batches), st, st + io.C,
+                                    partial.data_ptr<float>(), (int)partial.size(1), (float)eps, (float)momentum, relu, cur_stream());
+    return std::make_tuple(io.y, io.stats, io.mask);
   });
   m.def("bn_backward_partials", [](at::Tensor dy, at::Tensor x, c10::optional<at::Tensor> y, at::Tensor gamma, at::Tensor stats, bool relu,
                                    bool need_dres, at::Tensor partial) {
-    check_cuda(dy, "dy"); check_cuda(partial, "partial");
-    c10::cuda::CUDAGuard guard(x.device());
-    const int C = (int)x.size(1);
-    const int R = (int)(x.numel() / C);
-    TORCH_CHECK(partial.scalar_type() == at::kFloat && partial.dim() == 3 && partial.size(0) == 2 && partial.size(2) == C && partial.is_contiguous(),
+    BnBackwardIo io = bn_backward_io("bn_backward_partials", dy, x, y, relu, need_dres, 2);   // dparams rows: dgamma, dbeta
+    check_cuda(partial, "partial");
+    TORCH_CHECK(partial.scalar_type() == at::kFloat && partial.dim() == 3 && partial.size(0) == 2 && partial.size(2) == io.C && partial.is_contiguous(),
                 "bn_backward_partials: partial sums must be fp32 [2, groups, C]");
-    TORCH_CHECK(dy.is_contiguous(at::MemoryFormat::ChannelsLast) && dy.sizes() == x.sizes() && dy.dtype() == x.dtype(), "bn_backward_partials: dy must match x");
-    at::Tensor dx = at::empty_like(x);
-    at::Tensor dres = need_dres ? at::empty_like(x) : at::Tensor();
-    at::Tensor dparams = at::empty({2, C}, x.options().dtype(at::kFloat));   // rows: dgamma, dbeta
-    float* dp = dparams.data_ptr<float>();
+    TORCH_CHECK(dy.is_contiguous(at::MemoryFormat::ChannelsLast) && dy.sizes() == x.sizes() && dy.dtype() == x.dtype(),
+                "bn_backward_partials: dy must match x");
+    c10::cuda::CUDAGuard guard(x.device());
+    float* dp = io.dparams.data_ptr<float>();
     const float* st = stats.data_ptr<float>();
-    TORCH_CHECK(!relu || (y.has_value() && y->scalar_type() == at::kByte), "bn_backward_partials: needs the ReLU bitmask written by bn_forward");
-    launch_bn_backward_from_partials(dy.data_ptr(), x.data_ptr(), relu ? y->data_ptr() : nullptr, dx.data_ptr(), need_dres ? dres.data_ptr() : nullptr,
-                                     dtype_of(x), R, C, gamma.data_ptr<float>(), st, st + C, dp, dp + C, partial.data_ptr<float>(), (int)partial.size(1),
-                                     relu, cur_stream());
-    return std::make_tuple(dx, dres, dparams);
+    launch_bn_backward_from_partials(dy.data_ptr(), x.data_ptr(), io.relu_mask, io.dx.data_ptr(), need_dres ? io.dres.data_ptr() : nullptr,
+                                     dtype_of(x), io.R, io.C, gamma.data_ptr<float>(), st, st + io.C, dp, dp + io.C,
+                                     partial.data_ptr<float>(), (int)partial.size(1), relu, cur_stream());
+    return std::make_tuple(io.dx, io.dres, io.dparams);
   });
   m.def("bn_backward", [](at::Tensor dy, at::Tensor x, c10::optional<at::Tensor> y, at::Tensor gamma, at::Tensor stats, bool relu,
                           bool need_dres, at::Tensor partial, at::Tensor counters) {
-    check_cuda(dy, "dy");
+    BnBackwardIo io = bn_backward_io("bn_backward", dy, x, y, relu, need_dres, 4);   // dparams rows: dgamma, dbeta, coef1, coef2
     c10::cuda::CUDAGuard guard(x.device());
-    const int C = (int)x.size(1);
-    const int R = (int)(x.numel() / C);
     at::Tensor dyc = dy.is_contiguous(at::MemoryFormat::ChannelsLast) ? dy : dy.contiguous(at::MemoryFormat::ChannelsLast);
-    at::Tensor dx = at::empty_like(x);
-    at::Tensor dres = need_dres ? at::empty_like(x) : at::Tensor();
-    auto fopt = x.options().dtype(at::kFloat);
-    at::Tensor dparams = at::empty({4, C}, fopt);   // rows: dgamma, dbeta, coef1, coef2
-    float* dp = dparams.data_ptr<float>();
+    float* dp = io.dparams.data_ptr<float>();
     const float* st = stats.data_ptr<float>();
-    TORCH_CHECK(!relu || (y.has_value() && y->scalar_type() == at::kByte), "bn_backward: needs the ReLU bitmask written by bn_forward");
-    launch_bn_backward(dyc.data_ptr(), x.data_ptr(), relu ? y->data_ptr() : nullptr, dx.data_ptr(), need_dres ? dres.data_ptr() : nullptr,
-                       dtype_of(x), R, C, gamma.data_ptr<float>(), st, st + C, dp, dp + C, dp + 2 * C, partial.data_ptr<float>(),
+    launch_bn_backward(dyc.data_ptr(), x.data_ptr(), io.relu_mask, io.dx.data_ptr(), need_dres ? io.dres.data_ptr() : nullptr, dtype_of(x),
+                       io.R, io.C, gamma.data_ptr<float>(), st, st + io.C, dp, dp + io.C, dp + 2 * io.C, partial.data_ptr<float>(),
                        (unsigned int*)counters.data_ptr<int>(), relu, cur_stream());
-    return std::make_tuple(dx, dres, dparams);
+    return std::make_tuple(io.dx, io.dres, io.dparams);
   });
 
   // ---- max pooling ------------------------------------------------------------------------------

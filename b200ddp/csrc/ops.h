@@ -70,8 +70,6 @@ void launch_small_linear_bwd(const float* dy, const float* x, const float* w, co
 // ---------------- fused training BatchNorm (+residual) (+ReLU), channels_last (batchnorm.cu) --------------
 // x viewed as row-major [R = N*H*W, C]; C % 8 == 0; gamma/beta/statistics fp32.
 void bn_workspace_sizes(int R, int C, size_t* partial_floats, size_t* counters);
-// -1 = read B200DDP_PDL (default 0); 1 = statistics -> apply and bwd-reduce -> bwd-apply as programmatic dependent launches
-void set_bn_pdl(int on);
 void launch_bn_forward(const void* x, const void* residual, void* y, unsigned char* relu_mask /*[R, C/8] or null*/, DType dt, int R, int C, const float* gamma, const float* beta,
                        float* running_mean, float* running_var, long long* num_batches, float* save_mean, float* save_rstd,
                        float* scale, float* shift, float* partial, unsigned int* counters, float eps, float momentum, bool relu,
@@ -80,8 +78,8 @@ void launch_bn_forward(const void* x, const void* residual, void* y, unsigned ch
 // (written by the GEMM epilogue that produced x): finish kernel + apply kernel, x is read once instead of twice.
 void launch_bn_forward_from_partials(const void* x, const void* residual, void* y, unsigned char* relu_mask, DType dt, int R, int C,
                                      const float* gamma, const float* beta, float* running_mean, float* running_var,
-                                     long long* num_batches, float* save_mean, float* save_rstd, float* scale, float* shift,
-                                     const float* partial, int groups, float eps, float momentum, bool relu, cudaStream_t s);
+                                     long long* num_batches, float* save_mean, float* save_rstd, const float* partial, int groups,
+                                     float eps, float momentum, bool relu, cudaStream_t s);
 // Backward with S1 / S2 partial sums ([2][groups][C]) from the data-gradient epilogue of the consuming convolution: one launch
 // (reduce the partials per block, apply), no pass over dy and x for the reduction.
 void launch_bn_backward_from_partials(const void* dy, const void* x, const void* relu_mask, void* dx, void* dres, DType dt, int R, int C, const float* gamma,

@@ -28,7 +28,6 @@ run stem_pad8 B200DDP_STEM_PAD=8
 run conv1x1_tc B200DDP_CONV1X1_TC=1
 run conv1x1_tc_tmastore B200DDP_CONV1X1_TC=1 B200DDP_GEMM_TMA_STORE=1
 run conv1x1_tc_tmastore_bnfuse B200DDP_CONV1X1_TC=1 B200DDP_GEMM_TMA_STORE=1 B200DDP_CONV_BN_FUSE=1
-run bn_pdl B200DDP_PDL=1
 run conv3x3_tc B200DDP_CONV3X3_TC=1
-run all_conv_tc B200DDP_STEM_PAD=8 B200DDP_CONV1X1_TC=1 B200DDP_GEMM_TMA_STORE=1 B200DDP_CONV_BN_FUSE=1 B200DDP_CONV3X3_TC=1 B200DDP_PDL=1
+run all_conv_tc B200DDP_STEM_PAD=8 B200DDP_CONV1X1_TC=1 B200DDP_GEMM_TMA_STORE=1 B200DDP_CONV_BN_FUSE=1 B200DDP_CONV3X3_TC=1
 echo "== GEMM sweep (raster / TMA store variants)"; timeout 300 python bench/kernel_bench.py --only gemm --out $O/kernels_groupm.json > $O/kernels_groupm.log 2>&1; echo "rc=$?"; grep -i "gemm" $O/kernels_groupm.log | tail -n 60
